@@ -3,7 +3,7 @@
 
     audio-seconds / second (RTFx), tdt-ctc-110m, 10 s clips, 1/2/4/8 x B200
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 110m-64x10s|600m-16x30s]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 110m-64x10s|600m-16x30s] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" is one pass of the hot path (PCM -> log-mel -> FastConformer -> TDT greedy) over
@@ -32,6 +32,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -59,6 +60,17 @@ CONFIGS = {
 def valid_rows(rows):
     """(len, ids...) rows -> token lists (entries past len are not part of the row's value)."""
     return [r[1:1 + r[0]].tolist() for r in rows]
+
+
+def dump_tokens(dirname, arrs, n):
+    """Writes the token arrays of n utterances (what pk_fetch_tokens returns) as DIR/<name>.npy in float32, so that the
+    outputs of two builds can be compared; entries past an utterance's token count are -1."""
+    os.makedirs(dirname, exist_ok=True)
+    lens = arrs["len"][:n]
+    valid = np.arange(arrs["ids"].shape[1])[None, :] < lens[:, None]
+    np.save(os.path.join(dirname, "token_count.npy"), lens.astype(np.float32))
+    for name, key in (("token_ids", "ids"), ("token_start_frame", "start"), ("token_end_frame", "end"), ("token_confidence", "conf")):
+        np.save(os.path.join(dirname, name + ".npy"), np.where(valid, arrs[key][:n], -1).astype(np.float32))
 
 
 def peaks():
@@ -252,6 +264,8 @@ def run_stream_bench(args, conf):
     eng.sync()
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_tokens(args.dump_outputs, out[1], S)          # the tokens every stream emitted in the last timed step
     launches = eng.launch_count() - l0
     audio_s = S * K * CH / 16000.0
     value = audio_s / wall
@@ -315,8 +329,13 @@ def main():
     ap.add_argument("--config", default="110m-64x10s", choices=sorted(CONFIGS))
     ap.add_argument("--decoder", default="tdt", choices=["tdt", "ctc"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--tmp", default=os.environ.get("PK_BENCH_TMP", "/tmp/pk_bench"))
+    ap.add_argument("--tmp", default=os.environ.get("PK_BENCH_TMP", os.path.join(tempfile.gettempdir(), f"pk_bench_{os.getuid()}")),
+                    help="cache of the synthetic checkpoints (per user: the directory is shared by every run on the machine)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the token arrays of the last timed step as DIR/<name>.npy "
+                    "(float32; with N GPUs, those of rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps what the CUDA path computed (--impl ours)")
     os.makedirs(args.tmp, exist_ok=True)
     conf = CONFIGS[args.config]
     if args.steps is None:
@@ -432,6 +451,10 @@ def main():
     rows_all = eng.job_fetch(world * K * BATCH, gathered=True) if world > 1 else eng.job_fetch(K * BATCH)
     mine = rows_all[rank * K * BATCH:(rank + 1) * K * BATCH]
     assert int((rows_all[:, 0] > 0).sum()) == rows_all.shape[0], "bench: an utterance of the job decoded to nothing"
+    if args.dump_outputs and rank == 0:
+        last = eng.fetch_into(eng._tokens(BATCH))                  # micro-batch K - 1: the last timed step
+        assert valid_rows(np.concatenate([last["len"][:, None], last["ids"]], axis=1)) == valid_rows(mine[(K - 1) * BATCH:])
+        dump_tokens(args.dump_outputs, last, BATCH)
     eng.job_select(0, BATCH)
     eng.run_staged(dec)
     ref_tokens = eng.fetch(BATCH)                                  # micro-batch 0 again, through the plain token path

@@ -56,12 +56,6 @@ def synth(pkg):
     return s
 
 
-@pytest.fixture(scope="session")
-def refbind():
-    import refbind as R
-    return R if R.available() else None
-
-
 class Model:
     """A seeded synthetic checkpoint on disk + both config views + vocab."""
 
@@ -93,5 +87,16 @@ def m110(tmp_path_factory, pkg, O, synth):
 
 @pytest.fixture(scope="session")
 def golden():
-    p = os.path.join(ROOT, "tests", "golden", "golden_v1.npz")
-    return np.load(p, allow_pickle=False)
+    """The reference's outputs on the tiny model's clips and the 110m clip (two files, each below 1 MB)."""
+    d = {}
+    for name in ("golden_v1.npz", "golden_110m_v1.npz"):
+        with np.load(os.path.join(ROOT, "tests", "golden", name), allow_pickle=False) as z:
+            d.update(z)
+    return d
+
+
+@pytest.fixture(scope="session")
+def golden_refcalls():
+    """Single calls into the compiled reference that the oracle and resampler tests compare with."""
+    with np.load(os.path.join(ROOT, "tests", "golden", "golden_refcalls_v1.npz"), allow_pickle=False) as z:
+        return dict(z)

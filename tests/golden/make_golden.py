@@ -1,15 +1,16 @@
-"""Generates tests/golden/golden_v1.npz from the UNMODIFIED reference compiled here
-(oracle/_ref/libpkref.so <- /root/reference via oracle/Makefile).
+"""Generates the fixtures under tests/golden/ from the UNMODIFIED reference, compiled into
+oracle/_ref/libpkref.so by oracle/Makefile (REF=<path of the reference sources>).
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [boost|stream|refcalls|600m|600m_extra|600m_long|110m_extra]
 
 The reference ships no numeric golden vectors for mel / encoder (SURVEY.md section 4:
 its tests pin shapes and decode-loop logic only), so these are produced by running
 the reference itself on seeded synthetic checkpoints / audio
 (parakeet.cpp_b200/synth.py; same seeds as the tests' fixtures).  The fixtures pin
 oracle/oracle.py (tests/test_oracle.py, CPU) and the CUDA path (tests/test_gpu_parity.py).
-/root/reference is not needed to *consume* the fixtures.
+The reference is not needed to *consume* the fixtures.
 """
+import hashlib
 import os
 import sys
 import tempfile
@@ -91,9 +92,16 @@ def main():
     with tempfile.TemporaryDirectory() as td:
         run_model(out, "tiny", O.make_tiny_config(), 3, [(32000, 11), (20000, 12), (400, 13), (64000, 14)], td, True)
         run_model(out, "m110", O.make_110m_config(), 0, [(160000, 1000)], td, False)
-    path = os.path.join(ROOT, "tests", "golden", "golden_v1.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path) // 1024, "KiB")
+    # the 110m clip gets a file of its own (each fixture stays below 1 MB); its last layer is its encoder output,
+    # stored once as m110.c0.enc
+    k = "m110.c0."
+    assert np.array_equal(out[k + "layers_first_last"][1], out[k + "enc"])
+    out[k + "layer_first"] = out.pop(k + "layers_first_last")[0]
+    m110 = {n: out.pop(n) for n in list(out) if n.startswith("m110.")}
+    for name, d in (("golden_v1.npz", out), ("golden_110m_v1.npz", m110)):
+        path = os.path.join(ROOT, "tests", "golden", name)
+        np.savez_compressed(path, **d)
+        print("wrote", path, os.path.getsize(path) // 1024, "KiB")
 
 
 def main_600m():
@@ -272,6 +280,93 @@ def main_stream():
     print("wrote", path, os.path.getsize(path) // 1024, "KiB")
 
 
+def sha256(a):
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(a, np.float32).tobytes()).digest(), np.uint8)
+
+
+# the resampler inputs of tests/test_abi.py::test_resample_matches_oracle_and_reference (seed 4) and
+# tests/test_gpu_parity.py::test_gpu_resampler_matches_oracle_and_feeds_the_path (seed 9), drawn in the same order
+RESAMPLE_HOST = [(44100, 16000, 9000), (48000, 16000, 5001), (8000, 16000, 2500), (22050, 16000, 3000), (24000, 16000, 999),
+                 (96000, 16000, 6000), (16000, 16000, 50), (11025, 16000, 3), (16000, 8000, 1000), (44100, 16000, 0)]
+RESAMPLE_DEVICE = [(44100, 16000, [9000, 3, 20000]), (48000, 16000, [5001]), (8000, 16000, [2500, 1]), (22050, 16000, [30000, 12345]),
+                   (96000, 16000, [6000]), (16000, 8000, [1000]), (11025, 16000, [4097])]
+REF_STREAM_SCHEDULE = [2560, 3000, 800, 2560, 6000, 2560, 2560]
+
+
+def main_refcalls():
+    """What the oracle tests compare with single calls into the compiled reference: the tiny model's mel, subsampling,
+    per-layer encoder output and TDT decode of one 3 s clip; one tiny streaming model chunk by chunk; boosted CTC greedy
+    on random phrase sets; and parakeet::resample, stored as SHA-256 digests of its fp32 output (those comparisons
+    are bit-exact)."""
+    out = {}
+    with tempfile.TemporaryDirectory() as td:
+        ocfg = O.make_tiny_config()
+        W = synth.make_weights(ocfg, seed=3)
+        wp, vp = os.path.join(td, "tiny.safetensors"), os.path.join(td, "tiny.vocab.txt")
+        synth.save_safetensors(wp, W)
+        synth.save_vocab(vp, synth.make_vocab(ocfg.vocab - 1, seed=3))
+        m = R.RefModel(wp, vp, 0, cfg=ocfg)
+        n, aseed = 48000, 22
+        feats = R.mel(synth.make_audio(n, aseed))
+        sub, lay = m.encode_layers(feats, ocfg.d_model, ocfg.n_layers, O.encoder_len(feats.shape[0]))
+        out["tiny.n_samples"] = np.array([n, aseed], np.int64)
+        out["tiny.mel"], out["tiny.sub"], out["tiny.layers"] = feats, sub, lay
+        out["tiny.tdt_tok"], out["tiny.tdt_conf"] = toks_arr(m.tdt_greedy(lay[-1], True))
+        # boosted CTC greedy on the oracle's log-probs of golden clip 1
+        g = np.load(os.path.join(ROOT, "tests", "golden", "golden_v1.npz"))
+        lp = O.ctc_log_probs(W, g["tiny.c1.enc"])
+        rng = np.random.default_rng(23)
+        for i in range(5):
+            phrases = [rng.integers(0, ocfg.vocab - 1, size=int(rng.integers(1, 5))).tolist() for _ in range(8)]
+            k = f"boost.k{i}."
+            out[k + "clip"], out[k + "boost"] = np.array([1], np.int64), np.array([4.0], np.float32)
+            out[k + "ph_ids"] = np.array([t for ph in phrases for t in ph], np.int32)
+            out[k + "ph_len"] = np.array([len(ph) for ph in phrases], np.int32)
+            out[k + "ctc_tok"], _ = toks_arr(R.ctc_greedy_boosted(lp, ocfg.vocab - 1, phrases, 4.0))
+        out["boost.n_cases"] = np.array([5], np.int64)
+        m.close()
+        # streaming: the oracle first (the reference would hang on a livelocking decode)
+        scfg = O.make_tiny_stream_config()
+        wseed, aseed, sched = 9, 91, REF_STREAM_SCHEDULE
+        Ws = synth.make_weights(scfg, seed=wseed)
+        pcm = synth.make_audio(sum(sched), aseed)
+        pre, cache, st = O.StreamingPreprocessor(scfg.mel_bins), O.StreamEncoderCache(scfg.n_layers), O.StreamDecodeState(scfg)
+        pos = 0
+        for n in sched:
+            f = pre.process_chunk(pcm[pos:pos + n]); pos += n
+            e = O.stream_encoder_chunk(Ws, f, cache, scfg) if f is not None else None
+            if e is not None:
+                O.stream_decode_chunk(Ws, e, st, scfg, max_steps=5000)
+        wps = os.path.join(td, "tstream9.safetensors")
+        synth.save_safetensors(wps, Ws)
+        rs = R.RefStream(wps, scfg)
+        out["stream.seeds"], out["stream.schedule"] = np.array([wseed, aseed], np.int64), np.array(sched, np.int64)
+        pos = 0
+        for ci, n in enumerate(sched):
+            f, e, toks = rs.chunk(pcm[pos:pos + n]); pos += n
+            k = f"stream.k{ci}."
+            out[k + "feats"] = f if f is not None else np.zeros((0, scfg.mel_bins), np.float32)
+            out[k + "enc"] = e if e is not None else np.zeros((0, scfg.d_model), np.float32)
+            out[k + "tok"], _ = toks_arr(toks)
+        rs.close()
+    rng = np.random.default_rng(4)
+    for sr, dr, n in RESAMPLE_HOST:
+        x = (rng.standard_normal(n) * 0.3).astype(np.float32)
+        if n > 0:
+            out[f"resample_host.{sr}.{dr}.{n}.sha256"] = sha256(R.resample(x, sr, dr))
+    rng = np.random.default_rng(9)
+    for sr, dr, lens in RESAMPLE_DEVICE:
+        for n in lens:
+            x = (rng.standard_normal(n) * 0.3).astype(np.float32)
+            if n > 16:
+                y = R.resample(x, sr, dr)
+                assert np.array_equal(y, O.sinc_resample(x, sr, dr))      # the GPU test compares with the oracle's output
+                out[f"resample_device.{sr}.{dr}.{n}.sha256"] = sha256(y)
+    path = os.path.join(ROOT, "tests", "golden", "golden_refcalls_v1.npz")
+    np.savez_compressed(path, **out)
+    print("wrote", path, os.path.getsize(path) // 1024, "KiB")
+
+
 def boost_cases(vocab, base_ctc, rng):
     """Phrase sets for the boosted-decode fixtures: random short phrases plus one that continues a prefix of the
     unboosted output (so that deeper trie states are visited)."""
@@ -338,6 +433,8 @@ if __name__ == "__main__":
         main_boost()
     elif len(sys.argv) > 1 and sys.argv[1] == "stream":
         main_stream()
+    elif len(sys.argv) > 1 and sys.argv[1] == "refcalls":
+        main_refcalls()
     elif len(sys.argv) > 1 and sys.argv[1] == "600m_extra":
         main_600m_extra()
     elif len(sys.argv) > 1 and sys.argv[1] == "110m_extra":

@@ -1,10 +1,10 @@
 """CPU tests that PIN THE ORACLE (oracle/oracle.py) before it is trusted:
   (1) the reference's own known-answer tests that apply at this boundary
-      (/root/reference/tests/test_all.cpp: CTCDecode.* :759-872, PositionEmbedding.* :1003-1030,
+      (the reference's tests/test_all.cpp: CTCDecode.* :759-872, PositionEmbedding.* :1003-1030,
        GroupTimestamps.* / TimestampTypes.* :45-129, Tokenizer.DecodeOutOfRange :470-477),
-  (2) golden vectors produced by the unmodified reference compiled here
-      (tests/golden/golden_v1.npz <- tests/golden/make_golden.py),
-  (3) when oracle/_ref/libpkref.so is present, the live compiled reference.
+  (2) golden vectors produced by the unmodified reference
+      (tests/golden/golden_*.npz <- tests/golden/make_golden.py),
+  (3) recorded single calls into the compiled reference (tests/golden/golden_refcalls_v1.npz).
 """
 import os
 
@@ -163,24 +163,24 @@ def test_golden_110m_decode(O, synth, golden):
     assert O.detokenize([t[0] for t in ctc], pieces) == bytes(golden[k + "ctc_text"]).decode()
 
 
-# ---------------------------------------------------------------- (3) live compiled reference (when present)
-def test_live_reference_tiny(O, synth, refbind, tiny):
-    if refbind is None:
-        pytest.skip("oracle/_ref/libpkref.so not built")
-    m = refbind.RefModel(tiny.weights_path, tiny.vocab_path, 0, cfg=tiny.ocfg)
-    pcm = synth.make_audio(48000, 22)
-    fr = refbind.mel(pcm)
+# ---------------------------------------------------------------- (3) recorded calls into the compiled reference
+def test_live_reference_tiny(O, synth, tiny, golden_refcalls):
+    """The reference's mel, subsampling, per-layer encoder output and TDT decode of one 3 s clip (tiny model)."""
+    g = golden_refcalls
+    n, aseed = (int(v) for v in g["tiny.n_samples"])
+    pcm = synth.make_audio(n, aseed)
+    fr = g["tiny.mel"]
     fo = O.preprocess_audio(pcm)
     assert np.abs(fr - fo).max() < 2e-3
-    T = O.encoder_len(fr.shape[0])
-    sub_r, lay_r = m.encode_layers(fr, tiny.ocfg.d_model, tiny.ocfg.n_layers, T)
+    sub_r, lay_r = g["tiny.sub"], g["tiny.layers"]
+    assert lay_r.shape[1] == O.encoder_len(fr.shape[0])
     enc_o, sub_o, lay_o = O.encoder_forward(tiny.W, fr, tiny.ocfg, return_layers=True)
     assert _rel(sub_o, sub_r) < 2e-5
     for i in range(tiny.ocfg.n_layers):
         assert _rel(lay_o[i], lay_r[i]) < 5e-5
-    assert m.tdt_greedy(lay_r[-1], True)[:50] == [tuple(t) for t in O.tdt_greedy_decode(tiny.W, lay_r[-1], tiny.ocfg, with_timestamps=True)][:50] or \
-        [t[:3] for t in m.tdt_greedy(lay_r[-1], True)] == [t[:3] for t in O.tdt_greedy_decode(tiny.W, lay_r[-1], tiny.ocfg, with_timestamps=True)]
-    m.close()
+    ref_tdt = [(int(a), int(b), int(c), float(d)) for (a, b, c), d in zip(g["tiny.tdt_tok"], g["tiny.tdt_conf"])]
+    oracle_tdt = O.tdt_greedy_decode(tiny.W, lay_r[-1], tiny.ocfg, with_timestamps=True)
+    assert ref_tdt[:50] == [tuple(t) for t in oracle_tdt][:50] or [t[:3] for t in ref_tdt] == [tuple(t[:3]) for t in oracle_tdt]
 
 
 def test_golden_600m_decode(O, synth):
@@ -270,28 +270,23 @@ def test_streaming_context_mask_is_inert_in_the_reference(O, synth):
     assert worst > 1e-3
 
 
-def test_live_reference_streaming(O, synth, refbind, tmp_path):
-    if refbind is None:
-        pytest.skip("oracle/_ref/libpkref.so not built")
+def test_live_reference_streaming(O, synth, golden_refcalls):
+    """The reference's streaming path chunk by chunk on a second tiny streaming model, with uneven chunk sizes."""
+    g = golden_refcalls
     ocfg = O.make_tiny_stream_config()
-    W = synth.make_weights(ocfg, seed=9)
-    wp = str(tmp_path / "ts9.safetensors")
-    synth.save_safetensors(wp, W)
-    sched = [2560, 3000, 800, 2560, 6000, 2560, 2560]
-    pcm = synth.make_audio(sum(sched), 91)
-    want = _run_stream_oracle(O, synth, W, ocfg, pcm, sched)      # oracle first: the reference would hang on a livelock
-    rs = refbind.RefStream(wp, ocfg)
-    pos = 0
-    for n, (f, e, t) in zip(sched, want):
-        rf, re_, rt = rs.chunk(pcm[pos:pos + n])
-        pos += n
-        assert (rf is None) == (f is None) and (re_ is None) == (e is None)
+    wseed, aseed = (int(v) for v in g["stream.seeds"])
+    sched = [int(v) for v in g["stream.schedule"]]
+    W = synth.make_weights(ocfg, seed=wseed)
+    pcm = synth.make_audio(sum(sched), aseed)
+    for ci, (f, e, t) in enumerate(_run_stream_oracle(O, synth, W, ocfg, pcm, sched)):
+        k = f"stream.k{ci}."
+        rf, re_, rt = g[k + "feats"], g[k + "enc"], g[k + "tok"]      # (no rows: the reference returned nothing)
+        assert (len(rf) == 0) == (f is None) and (len(re_) == 0) == (e is None)
         if f is not None:
             assert _rel(f, rf) < 1e-4
         if e is not None:
             assert _rel(e, re_) < 1e-4
-        assert [x[:3] for x in rt] == [x[:3] for x in t]
-    rs.close()
+        assert rt.tolist() == [list(x[:3]) for x in t]
 
 
 # ------------------------------------------------------------------ phrase-boosted decode (SURVEY 8f row 3)
@@ -352,18 +347,17 @@ def test_golden_boosted_decode(O, synth, golden):
     assert len(g["enc.k0.ids"]) >= 4
 
 
-def test_live_reference_boosted_ctc(O, synth, refbind, golden):
-    if refbind is None:
-        pytest.skip("oracle/_ref/libpkref.so not built")
+def test_live_reference_boosted_ctc(O, synth, golden, golden_refcalls):
+    """The reference's boosted CTC greedy decode with random sets of eight phrases."""
+    g = golden_refcalls
     ocfg = O.make_tiny_config()
     W = synth.make_weights(ocfg, seed=3)
-    lp = O.ctc_log_probs(W, golden["tiny.c1.enc"])
-    rng = np.random.default_rng(23)
-    for _ in range(5):
-        phrases = [rng.integers(0, ocfg.vocab - 1, size=int(rng.integers(1, 5))).tolist() for _ in range(8)]
-        want = refbind.ctc_greedy_boosted(lp, ocfg.vocab - 1, phrases, 4.0)
-        got = O.ctc_greedy_decode_with_timestamps_boosted(lp, O.ContextTrie(phrases), 4.0, ocfg.vocab - 1)
-        assert [x[:3] for x in got] == [x[:3] for x in want]
+    for n in range(int(g["boost.n_cases"][0])):
+        k = f"boost.k{n}."
+        phrases, boost, ci = _boost_case(g, k)
+        lp = O.ctc_log_probs(W, golden[f"tiny.c{ci}.enc"])
+        got = O.ctc_greedy_decode_with_timestamps_boosted(lp, O.ContextTrie(phrases), boost, ocfg.vocab - 1)
+        assert [list(x[:3]) for x in got] == g[k + "ctc_tok"].tolist()
 
 
 def _boost_lp(pattern_or_none):
