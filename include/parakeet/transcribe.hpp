@@ -63,6 +63,8 @@ inline TDTConfig make_tdt_600m_config() {      // config.hpp:98-116
     c.prediction.vocab_size = 8193; c.joint.vocab_size = 8193;
     return c;
 }
+struct RNNTConfig { EncoderConfig encoder; PredictionConfig prediction; JointConfig joint; };
+inline RNNTConfig make_rnnt_600m_config() { return RNNTConfig{}; }   // config.hpp:119-135: the defaults above
 
 // ─── timestamps (timestamp.hpp:11-35) ────────────────────────────────────────
 struct TimestampedToken { int token_id; int start_frame; int end_frame; float confidence = 1.0f; };
@@ -247,7 +249,8 @@ class EngineHolder {
     EngineHolder(const pk_config &cfg, const std::string &weights, int device) : cfg_(cfg) {
         if (pk_engine_create(&cfg, weights.c_str(), device, &e_) != PK_OK)
             throw std::runtime_error(std::string("parakeet_b200: ") + pk_last_error(nullptr));
-        cap_ = 2 * pk_encoder_frames(pk_mel_frames(cfg.max_samples)) + 8;
+        const int32_t tmax = pk_encoder_frames(pk_mel_frames(cfg.max_samples));
+        cap_ = cfg.n_durations == 0 ? tmax * cfg.max_symbols : 2 * tmax + 8;     // (RNNT: up to max_symbols per frame)
     }
     EngineHolder(const EngineHolder &) = delete;
     EngineHolder &operator=(const EngineHolder &) = delete;
@@ -410,6 +413,32 @@ class TDTTranscriber : public detail::TranscriberBase<TDTTranscriber> {
         return TranscriberBase::transcribe(samples, o);
     }
     pk_decoder pick(Decoder) const { return PK_DECODER_TDT; }
+};
+
+/// RNNT models (rnnt-600m, reference config.hpp:119-135), with TDTTranscriber's surface.  The reference has no such
+/// class: its CLI does the same inline in run_rnnt_600m (src/main.cpp:296-360) -- preprocess_audio, the encoder, then
+/// rnnt_greedy_decode(_with_timestamps) with blank = vocab - 1.  Phrase boosting is not available for RNNT decoding.
+class RNNTTranscriber : public detail::TranscriberBase<RNNTTranscriber> {
+  public:
+    RNNTTranscriber(const std::string &weights_path, const std::string &vocab_path, const RNNTConfig &config = make_rnnt_600m_config(),
+                    int device = 0, int max_batch = 16, int max_samples = 30 * 16000) {
+        pk_config c;
+        pk_config_rnnt_600m(&c);
+        detail::fill(c, config.encoder, config.prediction, config.joint, {});
+        c.max_batch = max_batch; c.max_samples = max_samples;
+        eng_ = std::make_unique<detail::EngineHolder>(c, weights_path, device);
+        tokenizer_.load(vocab_path);
+    }
+    using TranscriberBase::transcribe;
+    TranscribeResult transcribe(const std::string &audio_path, bool timestamps = false) {
+        TranscribeOptions o; o.timestamps = timestamps;
+        return TranscriberBase::transcribe(audio_path, o);
+    }
+    TranscribeResult transcribe(const std::vector<float> &samples, bool timestamps = false) {
+        TranscribeOptions o; o.timestamps = timestamps;
+        return TranscriberBase::transcribe(samples, o);
+    }
+    pk_decoder pick(Decoder) const { return PK_DECODER_RNNT; }
 };
 
 

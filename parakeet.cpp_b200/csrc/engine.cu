@@ -278,7 +278,10 @@ pk_status pk_engine::load(const char *path) {
     const std::string jp = c.joint_prefix_tdt ? "tdt_joint_." : "joint_.";
     if ((s = make_weight(st, jp + "enc_proj_.weight", jp + "enc_proj_.bias", J, d, enc_proj))) return s;
     if ((s = get_vec(st, jp + "pred_proj_.weight", J * P, &Wp))) return s;
-    {
+    if (D == 0) {   // RNNTJoint (rnnt.cpp:34-45): one output head of V rows
+        if ((s = get_vec(st, jp + "out_proj_.weight", V * J, &Wout))) return s;
+        if ((s = get_vec(st, jp + "out_proj_.bias", V, &bout))) return s;
+    } else {
         std::vector<float> w((size_t)(V + D) * J), b((size_t)V + D), t;
         if (!st.read_f32(jp + "label_proj_.weight", t, (int64_t)V * J, e)) return fail(PK_ERR_MISSING, e);
         memcpy(w.data(), t.data(), t.size() * 4);
@@ -770,7 +773,8 @@ pk_status pk_engine::run_tdt() {
     TdtParams p{};
     p.P = c.pred_hidden; p.J = c.joint_hidden; p.V = c.vocab; p.D = c.n_durations; p.L = c.lstm_layers;
     p.Bpad = bp; p.n_utt = n_utt; p.cap = cap; p.n_dur = c.n_durations;
-    p.max_steps = maxT + cap + 2;
+    p.max_symbols = c.n_durations == 0 ? c.max_symbols : 0;
+    p.max_steps = maxT + cap + 2;     // (RNNT: every step emits or advances, so <= maxT + maxT * max_symbols steps)
     for (int i = 0; i < 8; ++i) p.durations[i] = c.durations[i];
     p.EP = EP; p.row_off = d_row_off; p.G0 = G0;
     for (int l = 0; l < c.lstm_layers; ++l) { p.Whh[l] = Whh_s[l]; p.Wih[l] = Wih_s[l]; p.bih[l] = bih[l]; }
@@ -893,6 +897,14 @@ void pk_config_tdt_600m(pk_config *c) {
     c->has_ctc = 0; c->joint_prefix_tdt = 0; c->max_batch = 16; c->max_samples = 480000;
 }
 
+void pk_config_rnnt_600m(pk_config *c) {
+    pk_config_110m(c);
+    c->d_model = 1024; c->n_layers = 24; c->ff = 4096; c->lstm_layers = 2;
+    c->n_durations = 0;
+    for (int i = 0; i < 8; ++i) c->durations[i] = 0;
+    c->has_ctc = 0; c->joint_prefix_tdt = 0; c->max_batch = 16; c->max_samples = 480000;
+}
+
 int32_t pk_mel_frames(int64_t n_samples) { return (int32_t)(1 + n_samples / 160); }
 int32_t pk_encoder_frames(int32_t f) { return conv_len(conv_len(conv_len(f))); }
 
@@ -915,7 +927,8 @@ pk_status pk_engine_create(const pk_config *cfg, const char *path, int device, p
     const pk_config &c = *cfg;
     if (c.d_model % 128 || c.d_model % c.n_heads || c.mel_bins % 8 || c.sub_channels % 4 || c.ff % 16 ||
         c.pred_hidden % 32 || c.joint_hidden % 32 || c.lstm_layers < 1 || c.lstm_layers > PK_MAX_LSTM ||
-        c.n_durations < 1 || c.n_durations > 8 || c.max_batch < 1 || c.max_samples < 400 || c.sub_channels > 1024) {
+        c.n_durations < 0 || c.n_durations > 8 || c.max_batch < 1 || c.max_samples < 400 || c.sub_channels > 1024 ||
+        (c.n_durations == 0 && (c.max_symbols < 1 || c.max_symbols > 64))) {
         g_create_err = "unsupported model shape in pk_config";
         return PK_ERR_INVALID;
     }
@@ -965,7 +978,8 @@ pk_status pk_engine_create(const pk_config *cfg, const char *path, int device, p
     e->f1n = conv_len(c.mel_bins);
     e->f2n = conv_len(e->f1n);
     e->f3n = conv_len(e->f2n);
-    e->cap = 2 * e->Tmax + 8;
+    // RNNT emits at most max_symbols tokens per frame, so Tmax * max_symbols can never truncate
+    e->cap = c.n_durations == 0 ? e->Tmax * c.max_symbols : 2 * e->Tmax + 8;
     pk_status s = e->load(path);
     if (s == PK_OK) s = e->alloc_workspace();
     if (s != PK_OK) {
@@ -1541,10 +1555,25 @@ static pk_status run_front(pk_engine *e) {
     e->front_done = true;
     return PK_OK;
 }
+// An RNNT engine (n_durations == 0) decodes with PK_DECODER_RNNT only, a TDT engine never does.
+static pk_status check_decoder(pk_engine *e, pk_decoder dec) {
+    if (dec != PK_DECODER_CTC && dec != PK_DECODER_TDT && dec != PK_DECODER_RNNT) return e->fail(PK_ERR_INVALID, "unknown pk_decoder");
+    const bool rnnt = e->cfg.n_durations == 0;
+    if (rnnt && dec != PK_DECODER_RNNT)
+        return e->fail(PK_ERR_INVALID, "this engine holds an RNNT model (n_durations = 0): decode with PK_DECODER_RNNT");
+    if (!rnnt && dec == PK_DECODER_RNNT)
+        return e->fail(PK_ERR_INVALID, "PK_DECODER_RNNT needs an RNNT model (pk_config.n_durations = 0)");
+    if (dec == PK_DECODER_RNNT && e->boost_on)
+        return e->fail(PK_ERR_INVALID, "phrase boosting is not available for RNNT decoding: clear it with pk_set_boost(e, ..., 0, ...)");
+    return PK_OK;
+}
+static pk_status run_decoder(pk_engine *e, pk_decoder dec) {    // the RNNT rule is a mode of the TDT decode kernel
+    return dec == PK_DECODER_CTC ? e->run_ctc(nullptr) : e->run_tdt();
+}
 static pk_status run_pipeline(pk_engine *e, pk_decoder dec) {   // everything after the front end
     pk_status s;
     if ((s = e->run_encoder(nullptr, nullptr))) return s;
-    return dec == PK_DECODER_CTC ? e->run_ctc(nullptr) : e->run_tdt();
+    return run_decoder(e, dec);
 }
 
 // The ~250 launches of one batch are replayed as ONE CUDA graph once a batch shape has been seen
@@ -1553,12 +1582,13 @@ pk_status pk_run_staged(pk_engine *e, pk_decoder dec) {
     if (!e || e->n_utt <= 0) return PK_ERR_INVALID;
     cudaSetDevice(e->device);
     if (e->gemm_err) return e->gemm_err;
+    if (pk_status ds = check_decoder(e, dec)) return ds;
     {
         pk_status fs = run_front(e);
         e->front_done = false;      // a second pk_run_staged of the same staged batch re-runs the front end
         if (fs) return fs;
     }
-    std::string key(1, dec == PK_DECODER_CTC ? 'c' : 't');
+    std::string key(1, dec == PK_DECODER_CTC ? 'c' : dec == PK_DECODER_RNNT ? 'r' : 't');
     const int32_t bg = e->boost_on ? e->boost_gen : 0;
     key.append(reinterpret_cast<const char *>(&bg), sizeof(bg));
     key.append(reinterpret_cast<const char *>(e->frame_off.data()), e->frame_off.size() * sizeof(int32_t));
@@ -1958,8 +1988,9 @@ pk_status pk_decode(pk_engine *e, const float *enc, const int32_t *enc_lens, int
     if (!e || !enc || !enc_lens) return PK_ERR_INVALID;
     cudaSetDevice(e->device);
     pk_status s;
+    if ((s = check_decoder(e, dec))) return s;
     if ((s = stage_enc(e, enc, enc_lens, n_utt))) return s;
-    if ((s = (dec == PK_DECODER_CTC ? e->run_ctc(nullptr) : e->run_tdt()))) return s;
+    if ((s = run_decoder(e, dec))) return s;
     return e->fetch(out);
 }
 

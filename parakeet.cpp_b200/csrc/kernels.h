@@ -171,6 +171,10 @@ void launch_ctc_collapse(const int32_t *best, const float *conf, const int32_t *
 // ------------------------------------------------------------------ tdt.cu (K10)
 struct TdtParams {
     int P, J, V, D, L, Bpad, n_utt, cap, max_steps, n_dur;
+    // RNNT mode (rnnt_greedy_decode(_with_timestamps), src/rnnt.cpp:56-177; D = 0, no duration head): blank advances one
+    // frame, a symbol stays on the frame (start = end = t), and the max_symbols-th symbol on a frame moves to the next
+    // frame with the state and token kept.  0 = TDT rule.
+    int max_symbols;
     int out_in_smem, wih_in_smem, smem_lstm_floats;   // filled by launch_tdt_decode
     int wstage_rows;                                  // rows of the shared-memory staging tile for weights that stay in L2 (0: none)
     int durations[8];

@@ -183,6 +183,7 @@ pk_status pk_stream_open(pk_engine *e, int32_t n_streams, int32_t max_chunk_samp
     cudaSetDevice(e->device);
     if (e->ss) return e->fail(PK_ERR_INVALID, "pk_stream_open: streams are already open on this engine");
     const pk_config &c = e->cfg;
+    if (c.n_durations == 0) return e->fail(PK_ERR_INVALID, "pk_stream_open: streaming is not available on an RNNT engine (n_durations = 0)");
     auto s = std::make_unique<StreamSet>();
     s->S = n_streams; s->L = att_context_left; s->R = att_context_right; s->max_chunk = max_chunk_samples;
     const int tot_max = 399 + max_chunk_samples;

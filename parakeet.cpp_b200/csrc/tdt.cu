@@ -17,6 +17,12 @@
 // symbols the inner loop is simply re-entered on the same frame with the same state), so it
 // is not modelled; a token capacity bounds the loop instead (reference would livelock).
 //
+// RNNT mode (p.max_symbols > 0, D = 0: rnnt_greedy_decode(_with_timestamps), src/rnnt.cpp:56-177) reuses every phase;
+// only the state update differs: blank -> state = saved, t += 1; symbol -> emit (start = end = t), token = symbol,
+// stay on the frame; the max_symbols-th symbol on one frame moves to the next frame with state and token KEPT.  The
+// per-utterance symbol count is replicated in shared memory like the frame position.  The engine sizes the token
+// capacity as Tmax * max_symbols, the most the rule can emit, so an RNNT decode is never truncated.
+//
 // Design (weights-stationary, 2-D decomposition): the grid is one CTA per SM, grouped in thread-block
 // CLUSTERS of CL = 4 (or 2) CTAs.  A cluster owns a block of weight ROWS (LSTM units, joint-hidden
 // rows, label/duration rows); inside the cluster, CTA rank q owns the K-SLICE [q K/CL, (q+1) K/CL) of
@@ -365,7 +371,8 @@ __global__ void __launch_bounds__(NTHR, 1) tdt_decode_kernel(TdtParams p) {
     int *s_token = s_cur + Bpad, *s_tpos = s_token + Bpad, *s_active = s_tpos + Bpad, *s_ntok = s_active + Bpad;
     int *s_pend = s_ntok + Bpad;                   // slot of a token whose confidence is still pending (-1: none)
     float *s_vraw = reinterpret_cast<float *>(s_pend + Bpad);   // raw (unboosted) logit of that token (phrase boosting)
-    bf16 *wbf = reinterpret_cast<bf16 *>(s_vraw + Bpad);
+    int *s_nsym = reinterpret_cast<int *>(s_vraw + Bpad);       // RNNT: symbols emitted on the current frame
+    bf16 *wbf = reinterpret_cast<bf16 *>(s_nsym + (p.max_symbols > 0 ? Bpad : 0));
     // Weight rows in global memory are [hi: K][lo: K]; a CTA keeps columns [k0, k0 + KS) of its cluster's rows.
     auto stage_rows = [&](bf16 *dst, const bf16 *src, int rows, int K, int k0, int KS) {
         const int RS = 2 * (KS + 4), n8 = KS / 4;            // 8-byte pieces per half row
@@ -435,6 +442,7 @@ __global__ void __launch_bounds__(NTHR, 1) tdt_decode_kernel(TdtParams p) {
         s_active[b] = (b < p.n_utt && p.row_off[b + 1] > p.row_off[b]) ? 1 : 0;
         s_ntok[b] = 0;
         s_pend[b] = -1;
+        if (p.max_symbols > 0) s_nsym[b] = 0;
     }
     __syncthreads();
     // Units this CTA finalises (same enumeration as the cell update in P1): pass ug, slot mi -> unit u, state slot cslot.
@@ -680,11 +688,14 @@ __global__ void __launch_bounds__(NTHR, 1) tdt_decode_kernel(TdtParams p) {
             unpack_key(p.key_lab[kb * KB + b], lmax, lidx);
             unpack_key(p.key_dur[kb * KB + b], dmax, didx);
             const int T = p.row_off[b + 1] - p.row_off[b];
-            const int skip = (didx < p.n_dur) ? p.durations[didx] : 1;
+            // (RNNT: no duration key; skip = 0 gives its rule below: blank t += 1, symbol end = start = t, stay)
+            const bool rnnt = p.max_symbols > 0;   // (read from the parameter here: no register held across the step)
+            const int skip = rnnt ? 0 : (didx < p.n_dur) ? p.durations[didx] : 1;
             int t = s_tpos[b];
             bool act = true;
             if (lidx == V - 1) {                 // blank: LSTM state reverts (cur unchanged)
                 t += max(skip, 1);
+                if (rnnt) s_nsym[b] = 0;
             } else {
                 const int n = s_ntok[b];
                 if (n < p.cap && (b % G) == g) { // the owner CTA writes the token; confidence follows
@@ -731,7 +742,12 @@ __global__ void __launch_bounds__(NTHR, 1) tdt_decode_kernel(TdtParams p) {
                 s_token[b] = lidx;
                 s_cur[b] = 1 - s_cur[b];         // commit the new LSTM state
                 t += skip;
-                if (n + 1 >= p.cap) {
+                if (rnnt) {                      // rnnt.cpp:82-106: the loop over max_symbols ends, the frame loop moves on
+                    const int ns = s_nsym[b] + 1;
+                    if (ns >= p.max_symbols) t += 1;
+                    s_nsym[b] = ns >= p.max_symbols ? 0 : ns;
+                }
+                if (n + 1 >= p.cap && !(rnnt && t >= T)) {   // (RNNT: a full buffer at the last frame is not a truncation)
                     act = false;
                     if ((b % G) == g) p.overflow[b] = 1;
                 }
@@ -819,7 +835,7 @@ size_t tdt_smem_bytes(const TdtParams &p, int n_clusters, int CL, bool *out_in_s
     const int KSmax = ge.KSP > ge.KSJ ? ge.KSP : ge.KSJ;
     const int xrows = p.Bpad < BCH ? p.Bpad : BCH;      // the x staging planes hold min(64, Bpad) utterance rows
     size_t fixed = (size_t)RG * RLD + (size_t)MYMAX * BCH + (size_t)2 * xrows * (KSmax + 8) / 2 + (size_t)p.L * 2 * ge.MU * p.Bpad +
-                   7 * (size_t)p.Bpad;
+                   (p.max_symbols > 0 ? 8 : 7) * (size_t)p.Bpad;
     // a staged weight row = [hi KS+4][lo KS+4] bf16 = KS + 4 floats
     const size_t hh = (size_t)p.L * ge.UPC * 4 * (ge.KSP + 4), ih = (size_t)(p.L - 1) * ge.UPC * 4 * (ge.KSP + 4);
     const size_t wp = (size_t)ge.JPC * (ge.KSP + 4), wo = (size_t)ge.OPC * (ge.KSJ + 4);

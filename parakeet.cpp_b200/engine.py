@@ -3,7 +3,7 @@ high-level API (include/parakeet/transcribe.hpp:23-190 in the reference):
 
     Transcriber(weights_path, vocab_path, config=make_110m_config())
     .to_gpu()
-    .transcribe(samples | path, decoder=Decoder.TDT, timestamps=False) -> TranscribeResult
+    .transcribe(samples | path, decoder=None (the model's default), timestamps=False) -> TranscribeResult
     .transcribe(samples | path, TranscribeOptions(...))
 
 plus `transcribe_batch`, which the reference lacks (it is batch-1 only,
@@ -41,7 +41,7 @@ class _PkTokens(C.Structure):
                 ("end", C.POINTER(C.c_int32)), ("conf", C.POINTER(C.c_float)), ("len", C.POINTER(C.c_int32))]
 
 
-EXPORTS = ["pk_config_110m", "pk_config_tdt_600m", "pk_engine_create", "pk_engine_destroy", "pk_last_error",
+EXPORTS = ["pk_config_110m", "pk_config_tdt_600m", "pk_config_rnnt_600m", "pk_engine_create", "pk_engine_destroy", "pk_last_error",
            "pk_mel_frames", "pk_encoder_frames", "pk_mel", "pk_encode", "pk_decode", "pk_ctc_logprobs",
            "pk_transcribe_batch", "pk_stage_pcm", "pk_prefetch_pcm", "pk_run_staged", "pk_fetch_tokens", "pk_sync",
            "pk_token_buffer", "pk_stream", "pk_launch_count", "pk_profile_begin", "pk_profile_end",
@@ -69,6 +69,7 @@ def load_library():
     vp, i32p, f32p, i64p = C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_float), C.POINTER(C.c_int64)
     L.pk_config_110m.argtypes = [C.POINTER(_PkConfig)]
     L.pk_config_tdt_600m.argtypes = [C.POINTER(_PkConfig)]
+    L.pk_config_rnnt_600m.argtypes = [C.POINTER(_PkConfig)]
     L.pk_engine_create.argtypes = [C.POINTER(_PkConfig), C.c_char_p, C.c_int, C.POINTER(vp)]
     L.pk_engine_destroy.argtypes = [vp]
     L.pk_last_error.argtypes = [vp]
@@ -156,7 +157,8 @@ class ModelConfig:
     pred_hidden: int = 640
     lstm_layers: int = 1
     joint_hidden: int = 640
-    durations: tuple = (0, 1, 2, 3, 4)
+    durations: tuple = (0, 1, 2, 3, 4)    # () = RNNT joint (one "out_proj_" head, decoded with Decoder.RNNT)
+    max_symbols: int = 10                 # max_symbols_per_step (tdt.hpp, rnnt.hpp); an RNNT engine holds this many tokens per frame
     has_ctc: bool = True
     joint_prefix: str = "tdt_joint_."
     name: str = "tdt-ctc-110m"
@@ -178,9 +180,13 @@ class ModelConfig:
             c.durations[i] = d
         c.has_ctc = int(self.has_ctc)
         c.joint_prefix_tdt = int(self.joint_prefix == "tdt_joint_.")
-        c.max_symbols = 10
+        c.max_symbols = self.max_symbols
         c.max_batch, c.max_samples, c.math = self.max_batch, self.max_samples, int(self.math)
         return c
+
+    @property
+    def is_rnnt(self) -> bool:
+        return len(self.durations) == 0
 
 
 def make_110m_config(**kw) -> ModelConfig:           # config.hpp:77-95
@@ -190,6 +196,22 @@ def make_110m_config(**kw) -> ModelConfig:           # config.hpp:77-95
 def make_tdt_600m_config(**kw) -> ModelConfig:       # config.hpp:98-116
     base = dict(mel_bins=128, d_model=1024, n_layers=24, ff=4096, vocab=8193, lstm_layers=2, has_ctc=False,
                 joint_prefix="joint_.", name="tdt-600m", max_batch=16, max_samples=480000)
+    base.update(kw)
+    return ModelConfig(**base)
+
+
+def make_rnnt_600m_config(**kw) -> ModelConfig:      # config.hpp:119-135 (80 mels into d 1024: proj_ is 2560 -> 1024)
+    base = dict(d_model=1024, n_layers=24, ff=4096, vocab=1025, lstm_layers=2, durations=(), has_ctc=False,
+                joint_prefix="joint_.", name="rnnt-600m", max_batch=16, max_samples=480000)
+    base.update(kw)
+    return ModelConfig(**base)
+
+
+def make_tiny_rnnt_config(**kw) -> ModelConfig:
+    """Small test-only RNNT shape (tiny encoder, 2 LSTM layers; not a reference preset)."""
+    base = dict(sub_channels=64, d_model=128, n_layers=2, n_heads=2, ff=256, vocab=33, pred_hidden=64, lstm_layers=2,
+                joint_hidden=64, durations=(), has_ctc=False, joint_prefix="joint_.", name="tiny-rnnt", max_batch=8,
+                max_samples=64000)
     base.update(kw)
     return ModelConfig(**base)
 
@@ -222,6 +244,7 @@ def make_tiny_config(**kw) -> ModelConfig:
 class Decoder(enum.IntEnum):          # transcribe.hpp:34
     CTC = 0
     TDT = 1
+    RNNT = 2                          # rnnt_greedy_decode(_with_timestamps), rnnt.cpp:56-177: RNNT models only
 
 
 @dataclass
@@ -250,7 +273,7 @@ class TranscribeResult:               # transcribe.hpp:23-30
 
 @dataclass
 class TranscribeOptions:              # transcribe.hpp:38-43
-    decoder: Decoder = Decoder.TDT
+    decoder: Optional[Decoder] = None     # None: the model's default (TDT; RNNT for an RNNT model)
     timestamps: bool = False
     boost_phrases: List[str] = field(default_factory=list)
     boost_score: float = 5.0
@@ -360,7 +383,7 @@ class Engine:
         if st != 0:
             raise RuntimeError(f"pk_engine_create failed ({st}): " + self.L.pk_last_error(None).decode())
         self.Tmax = self.L.pk_encoder_frames(self.L.pk_mel_frames(cfg.max_samples))
-        self.cap = 2 * self.Tmax + 8
+        self.cap = self.Tmax * cc.max_symbols if cfg.is_rnnt else 2 * self.Tmax + 8   # tokens per utterance, as pk_engine_create sizes them
 
     def close(self):
         if self.h:
@@ -692,7 +715,9 @@ def ctc_greedy_decode_boosted(logprobs: np.ndarray, phrases: Sequence[Sequence[i
 
 
 class Transcriber:
-    """Python mirror of parakeet::Transcriber / TDTTranscriber (transcribe.hpp:55-299)."""
+    """Python mirror of parakeet::Transcriber / TDTTranscriber (transcribe.hpp:55-299).  With an RNNT config
+    (make_rnnt_600m_config) the default decoder is Decoder.RNNT, the model's only one; asking such a model for CTC or TDT
+    raises ValueError, as the C-ABI rejects it."""
 
     def __init__(self, weights_path: str, vocab_path: str, config: Optional[ModelConfig] = None, device: int = 0):
         self.config = config or make_110m_config()
@@ -715,7 +740,16 @@ class Transcriber:
                 r.word_timestamps = self.tokenizer.group_words(toks)
         return r
 
-    def transcribe(self, audio, decoder=Decoder.TDT, timestamps: bool = False) -> TranscribeResult:
+    def _decoder(self, decoder: Optional[Decoder]) -> Decoder:
+        if self.config.is_rnnt:
+            if decoder is not None and decoder != Decoder.RNNT:
+                raise ValueError(f"{self.config.name} is an RNNT model: it decodes with Decoder.RNNT only")
+            return Decoder.RNNT
+        if decoder is None:
+            return Decoder.TDT
+        return decoder if self.config.has_ctc else Decoder.TDT
+
+    def transcribe(self, audio, decoder: Optional[Decoder] = None, timestamps: bool = False) -> TranscribeResult:
         if isinstance(decoder, TranscribeOptions):
             opts = decoder
         else:
@@ -723,13 +757,14 @@ class Transcriber:
         if opts.boost_phrases:
             raise NotImplementedError("phrase boosting is outside the B200 hot path (SURVEY.md section 8f.3)")
         samples = read_wav(audio) if isinstance(audio, str) else np.asarray(audio, np.float32)
-        dec = opts.decoder if self.config.has_ctc else Decoder.TDT
+        dec = self._decoder(opts.decoder)
         toks = self.engine.transcribe_batch([samples], dec)[0]
         return self._result(toks, opts.timestamps)
 
-    def transcribe_batch(self, audios, decoder=Decoder.TDT, timestamps: bool = False) -> List[TranscribeResult]:
+    def transcribe_batch(self, audios, decoder: Optional[Decoder] = None, timestamps: bool = False) -> List[TranscribeResult]:
         pcms = [read_wav(a) if isinstance(a, str) else np.asarray(a, np.float32) for a in audios]
         out = []
+        decoder = self._decoder(decoder) if (self.config.is_rnnt or decoder is None) else decoder
         B = self.config.max_batch
         for i in range(0, len(pcms), B):
             for toks in self.engine.transcribe_batch(pcms[i:i + B], decoder):

@@ -69,10 +69,13 @@ def tensor_specs(cfg):
               (q + "hidden_proj_.weight", (4 * P, P), "w")]
     j = cfg.joint_prefix
     s += [(j + "enc_proj_.weight", (J, d), "w"), (j + "enc_proj_.bias", (J,), "b"),
-          (j + "pred_proj_.weight", (J, P), "w"),
-          (j + "label_proj_.weight", (V, J), "head"), (j + "label_proj_.bias", (V,), "lab_b"),
-          (j + "duration_proj_.weight", (len(cfg.durations), J), "head"),
-          (j + "duration_proj_.bias", (len(cfg.durations),), "dur_b")]
+          (j + "pred_proj_.weight", (J, P), "w")]
+    if len(cfg.durations) == 0:         # RNNTJoint (rnnt.cpp:34-45): one output head, no durations
+        s += [(j + "out_proj_.weight", (V, J), "head"), (j + "out_proj_.bias", (V,), "lab_b")]
+    else:
+        s += [(j + "label_proj_.weight", (V, J), "head"), (j + "label_proj_.bias", (V,), "lab_b"),
+              (j + "duration_proj_.weight", (len(cfg.durations), J), "head"),
+              (j + "duration_proj_.bias", (len(cfg.durations),), "dur_b")]
     return s
 
 
